@@ -3,7 +3,7 @@
 metric 1, SURVEY.md §8d) on config C2: 100 000 pods x 1 000 templates, resources + taints/tolerations,
 and the scale-up decision latency (metric 2) beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2] [--dump-outputs DIR]
 
 One "step" = one dense pass of the scale-up predicate path over the whole pending-pod batch:
 every pod (not only group exemplars) against every template through the Filter chain.
@@ -167,6 +167,29 @@ def _cpu_dense(pool, procs, p_range, t_range):
 
 def _spread(n, k):
     return sorted({int(round(i * (n - 1) / max(k - 1, 1))) for i in range(k)})
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, fit_bits, P, fit_count):
+    """Writes what a caller of the dense pass receives, within DUMP_BYTES in all:
+      fit.npy       float32 [T][n]  1.0 = pod fit_pods[j] fits template t, else 0.0 (unpacked from fit_bits [T][ceil(P/32)]),
+                                    so one wrong verdict is an absolute difference of 1 under any tolerance
+      fit_pods.npy  float64 [n]     the pods kept: all P, or above the budget a fixed seeded sample, in ascending order
+      fit_count.npy float64 [T]     the fit histogram
+    With several ranks, fit covers rank 0's pod shard only (pods 0 .. P-1 of the snapshot) while fit_count counts the pods
+    of every rank, so fit_count is not the row sum of fit."""
+    T = fit_bits.shape[0]
+    room = (DUMP_BYTES - 4096 - 8 * T) // (4 * T + 8) if T else P       # 4096: the three .npy headers
+    if P and room < 1:
+        raise ValueError("--dump-outputs: one pod column of %d templates exceeds %d bytes" % (T, DUMP_BYTES))
+    pods = np.arange(P) if P <= room else np.sort(np.random.default_rng(0).choice(P, room, replace=False))
+    fit = (fit_bits[:, pods >> 5] >> (pods & 31).astype(np.uint32)) & 1
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "fit.npy"), fit.astype(np.float32))
+    np.save(os.path.join(path, "fit_pods.npy"), pods.astype(np.float64))
+    np.save(os.path.join(path, "fit_count.npy"), np.asarray(fit_count, np.float64))
 
 
 def reference_arm(args, cfg, P1, T, metric):
@@ -369,7 +392,12 @@ def main():
     ap.add_argument("--no-decision", action="store_true", help="engine arm: skip the decision-latency figures")
     ap.add_argument("--collective", default="peer", choices=["peer", "nccl"],
                     help="N>1: how the int32[T] fit histogram is reduced: fused P2P exchange in the kernel's last block, or NCCL")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="engine arm: write the results of the last timed step (rank 0's fit verdicts, the fit histogram over all "
+                         "ranks) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -448,12 +476,17 @@ def main():
                 dist.all_reduce(sync_t)                        # device-side barrier on the engine's stream: the ranks' timed
                                                                # windows open together (a host barrier cannot align queued work)
 
-    def step_resident():
-        eng.lib.cae_feasibility(eng.h, None, None, None)       # kernel only; results stay in HBM
+    def step_resident(to_host=False):
+        if to_host:                                            # the same launch; the copies of its results to the host
+            out = eng.feasibility()                            # are queued after its timing events
+        else:
+            eng.lib.cae_feasibility(eng.h, None, None, None)   # kernel only; results stay in HBM
+            out = None
         if count_t is not None:
             ar0.record()
             dist.all_reduce(count_t)                           # int32[T] histogram over NVLink
             ar1.record()
+        return out
 
     sampler = _clock_sampler_start([local_rank]) if rank == 0 else None   # rank 0's GPU only: NVML queries delay launches
     first_sample = None
@@ -469,21 +502,24 @@ def main():
         dist.barrier()
     for _ in range(args.warmup):   # warm-up AFTER the wait above: the GPUs idled while nvidia-smi initialised
         flush_l2()
-        step_resident()
+        step_resident(to_host=bool(args.dump_outputs))        # allocates the pinned result buffers the dumped step reuses
     torch.cuda.synchronize()
     launches0 = eng.stats().kernel_launches
     dev_ms, wall_ms, ar_ms = [], [], []
-    for _ in range(args.steps):
+    for s in range(args.steps):
         torch.cuda.synchronize()
         if dist is not None:
             dist.barrier()
         flush_l2()                                             # L2 flush between timed iterations (untimed, same stream)
-        step_resident()
+        out = step_resident(to_host=bool(args.dump_outputs) and s == args.steps - 1)
         torch.cuda.synchronize()
         dev_ms.append(eng.stats().feasibility_ms)
         if count_t is not None:
             ar_ms.append(ar0.elapsed_time(ar1))
     launches = eng.stats().kernel_launches - launches0
+    if args.dump_outputs and rank == 0:
+        bits, _, cnt = out
+        dump_outputs(args.dump_outputs, bits, Pl, count_t.cpu().numpy() if count_t is not None else cnt)
     for _ in range(10):                                        # host view of a step: launch + device + synchronize
         torch.cuda.synchronize()
         t0 = time.perf_counter()

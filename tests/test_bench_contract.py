@@ -1,21 +1,68 @@
-"""bench.py's reference arm runs without a GPU: its JSON line must carry the contract's keys, the SAME config dict the engine
-arm prints (the driver compares them), and the parity / decision legs must answer through the oracle."""
+"""bench.py's reference arm runs without a GPU: its JSON line must carry the benchmark's keys, the SAME config dict the engine
+arm prints (both lines describe one workload), and the parity / decision legs must answer through the oracle.  The engine
+arm's --dump-outputs writes what its last timed step computed."""
 import json
 import os
 import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def _ref(*extra):
+def _bench(*args, timeout=300):
     env = {k: v for k, v in os.environ.items() if k not in ("RANK", "WORLD_SIZE", "LOCAL_RANK")}
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--pods", "3000", "--templates", "24"] + list(extra),
-                         capture_output=True, text=True, timeout=300, env=env)
+    return subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + list(args), capture_output=True, text=True,
+                          timeout=timeout, env=env)
+
+
+def _ref(*extra):
+    out = _bench("--impl", "reference", "--pods", "3000", "--templates", "24", *extra)
     assert out.returncode == 0, out.stderr[-2000:]
     return json.loads(out.stdout.strip().splitlines()[-1])
+
+
+def test_steps_must_be_positive():
+    out = _bench("--impl", "reference", "--steps", "0")
+    assert out.returncode == 2 and "--steps" in out.stderr
+
+
+def test_dump_outputs_unpacks_and_samples_pods_above_the_budget(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    from kubernetes_autoscaler_b200.engine import unpack_bits
+    rng = np.random.default_rng(1)
+    small = rng.integers(0, 2 ** 32, (24, 94), dtype=np.uint32)
+    bench.dump_outputs(str(tmp_path / "small"), small, 3000, np.arange(24, dtype=np.int32))
+    fit = np.load(tmp_path / "small" / "fit.npy")
+    assert fit.dtype == np.float32 and np.array_equal(fit, unpack_bits(small, 3000))
+    assert np.array_equal(np.load(tmp_path / "small" / "fit_pods.npy"), np.arange(3000))
+    big = rng.integers(0, 2 ** 32, (200, 3125), dtype=np.uint32)           # 200 x 100 000 verdicts = 80 MB as float32
+    bench.dump_outputs(str(tmp_path / "big"), big, 100_000, np.arange(200, dtype=np.int32))
+    assert sum(f.stat().st_size for f in (tmp_path / "big").iterdir()) <= bench.DUMP_BYTES
+    pods = np.load(tmp_path / "big" / "fit_pods.npy").astype(np.int64)
+    assert len(pods) > 79_000 and np.all(np.diff(pods) > 0) and pods[-1] < 100_000
+    assert np.array_equal(np.load(tmp_path / "big" / "fit.npy"), unpack_bits(big, 100_000)[:, pods])
+    assert np.array_equal(np.load(tmp_path / "big" / "fit_count.npy"), np.arange(200))
+    with pytest.raises(ValueError):                                       # not even one pod column of every template fits
+        bench.dump_outputs(str(tmp_path / "huge"), np.broadcast_to(np.uint32(0), (20_000_000, 1)), 32, np.zeros(1))
+
+
+@pytest.mark.gpu
+def test_engine_arm_dumps_its_last_step(tmp_path, oracle):
+    from kubernetes_autoscaler_b200 import synth
+    out = _bench("--pods", "3000", "--templates", "24", "--steps", "3", "--warmup", "3", "--no-decision",
+                 "--dump-outputs", str(tmp_path), timeout=900)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads(out.stdout.strip().splitlines()[-1])
+    assert d["steps"] == 3 and len(d["step_ms_rank0"]) == 3 and d["parity_checked"]
+    want, _ = oracle.feasibility_dense(synth.generate(2, pods=3000, templates=24))
+    fit = np.load(tmp_path / "fit.npy")
+    assert fit.dtype == np.float32 and np.array_equal(fit, want == 0)
+    assert np.array_equal(np.load(tmp_path / "fit_count.npy"), (want == 0).sum(axis=1))
+    assert np.array_equal(np.load(tmp_path / "fit_pods.npy"), np.arange(3000))
 
 
 def test_reference_arm_line():

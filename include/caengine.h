@@ -361,6 +361,36 @@ int32_t cae_filter_schedulable(cae_engine* e, const int32_t* pod_order, int32_t 
                                int32_t last_index_in, int32_t break_on_failure, int32_t* assigned_node,
                                int32_t* last_index_out, int32_t* overflowing_controllers);
 
+/* The scale-down consumer of the same pass, batched: the planner's loop over the unneeded-node candidates of a tick
+ * (categorizeNodes, core/scaledown/planner/planner.go) calling RemovalSimulator.SimulateNodeRemoval (simulator/cluster.go:126-217)
+ * for each one in turn, on ONE snapshot, in one call.  Candidate c leaves the snapshot (its residents, DaemonSet pods
+ * included, stop counting for topology spread / inter-pod affinity), its pods are tried by HintingSimulator.TrySchedulePods
+ * with breakOnFailure on the remaining nodes (findPlaceFor, :184-217), and it is removable iff every pod is placed.
+ *   cand_node [n_cand]         cluster node index of each candidate, in the planner's order
+ *   cand_pod_off [n_cand+1], cand_pods   pending-pod indices of each candidate's pods to move (GetPodsToMove), in order; the
+ *                              pending rows of the last cae_load are these pods with nodeName cleared (its templates are ignored);
+ *                              a pod may be listed under one candidate only
+ *   hint_node [num_pending]    Hints.Get of each pod as a cluster node index, -1 = none; NULL = no hints.  A hint naming a
+ *                              node out of the snapshot is ignored, like a hint naming a deleted node (hinting_simulator.go:88-91)
+ *   node_ok [N]                the destination map (nodes the pods may go to), NULL = every node
+ *   persist                    persistSuccessfulSimulations: a removable candidate stays removed and its pods stay where they
+ *                              were placed for the rest of the call (withForkedSnapshot Commit, :169-182); pods placed on a later
+ *                              candidate are then part of ITS pods to move, after its own, in placement order.  Any other
+ *                              simulation is reverted.  The loaded snapshot itself never changes.
+ *   max_removable              unneededNodesLimit: once that many candidates are removable the rest are not simulated; 0 = no limit
+ *   last_index_in              SchedulerPluginRunner.lastIndex before the loop (raw, >= 0); ONE runner serves every simulation
+ * Outputs: result [n_cand] 0 removable, 1 NoPlaceToMovePods, 2 NoNodeInfo (removed by an earlier persisted simulation, or
+ * listed twice), -1 not simulated (after max_removable).  The trace: trace_off [n_cand+1] into trace_pod / trace_node
+ * [trace_cap]: for every simulated candidate the exact pod list TrySchedulePods received (NodeToBeRemoved.PodsToReschedule)
+ * and the node each pod went to, -1 = not placed or not tried after the first failure; the caller sets its hints from it.
+ * last_index_out: the runner's lastIndex after the loop.
+ * Status 1: the trace needs more than trace_cap entries (the message names it; a trace never needs more than
+ * n_cand x num_pending) or the placement log overflowed; -2: malformed input.  No other engine result changes. */
+int32_t cae_simulate_removals(cae_engine* e, int32_t n_cand, const int32_t* cand_node, const int32_t* cand_pod_off,
+                              const int32_t* cand_pods, const int32_t* hint_node, const uint8_t* node_ok, int32_t persist,
+                              int32_t max_removable, int32_t last_index_in, int32_t* result, int32_t trace_cap, int32_t* trace_off,
+                              int32_t* trace_pod, int32_t* trace_node, int32_t* last_index_out);
+
 /* The two halves of cae_expander_best for templates sharded over ranks (no [T][E] matrix ever leaves a GPU):
  * cae_waste_scores returns the least-waste score (expander/waste/waste.go:44-72) of this rank's template shard from
  * the device-resident result of the last cae_estimate_all, 0.0 for the rows of other ranks, so that a SUM all-reduce of

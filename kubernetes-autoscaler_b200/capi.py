@@ -162,6 +162,9 @@ def load_engine_lib() -> C.CDLL:
     lib.cae_filter_schedulable.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                            C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.cae_filter_schedulable.restype = C.c_int32
+    lib.cae_simulate_removals.argtypes = [C.c_void_p, C.c_int32] + [C.c_void_p] * 5 + [C.c_int32] * 3 + [C.c_void_p, C.c_int32] + \
+        [C.c_void_p] * 4
+    lib.cae_simulate_removals.restype = C.c_int32
     lib.cae_price_scores.argtypes = [C.c_void_p, P(cae_price_inputs), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.cae_price_scores.restype = C.c_int32
     lib.cae_expander_chain_ex.argtypes = [C.c_void_p, C.c_int32, C.c_int32] + [C.c_void_p] * 7

@@ -1034,6 +1034,152 @@ int32_t cae_filter_schedulable(cae_engine* h, const int32_t* pod_order, int32_t 
   return 0;
 }
 
+int32_t cae_simulate_removals(cae_engine* h, int32_t n_cand, const int32_t* cand_node, const int32_t* cand_pod_off,
+                              const int32_t* cand_pods, const int32_t* hint_node, const uint8_t* node_ok, int32_t persist,
+                              int32_t max_removable, int32_t last_index_in, int32_t* result, int32_t trace_cap, int32_t* trace_off,
+                              int32_t* trace_pod, int32_t* trace_node, int32_t* last_index_out) {
+  Engine* e = reinterpret_cast<Engine*>(h);
+  if (!e || !e->loaded) { cae::set_error("cae_simulate_removals before cae_load"); return -2; }
+  auto bad = [](const char* what) { cae::set_error(std::string("cae_simulate_removals: ") + what); return -2; };
+  if (n_cand < 0 || trace_cap < 0 || max_removable < 0 || last_index_in < 0 || !trace_off || !last_index_out ||
+      (n_cand > 0 && (!cand_node || !cand_pod_off || !result)) || (trace_cap > 0 && (!trace_pod || !trace_node)))
+    return bad("bad arguments");
+  cudaSetDevice(e->cfg.device);
+  const int P = e->P, N = e->N;
+  if (n_cand == 0) { trace_off[0] = 0; *last_index_out = last_index_in; return 0; }
+  if (cand_pod_off[0] != 0) return bad("cand_pod_off[0] must be 0");
+  for (int c = 0; c < n_cand; ++c) {
+    if (cand_node[c] < 0 || cand_node[c] >= N) return bad("candidate node index out of range");
+    if (cand_pod_off[c + 1] < cand_pod_off[c]) return bad("cand_pod_off is not monotone");
+  }
+  const int n_pods = cand_pod_off[n_cand];
+  if (n_pods > 0 && !cand_pods) return bad("bad arguments");
+  std::vector<uint8_t> listed(std::max(P, 1), 0);
+  for (int k = 0; k < n_pods; ++k) {
+    const int pod = cand_pods[k];
+    if (pod < 0 || pod >= P) return bad("pod index out of range");
+    if (listed[pod]) return bad("a pod is listed under two candidates");
+    listed[pod] = 1;
+  }
+  if (hint_node)
+    for (int i = 0; i < P; ++i)
+      if (hint_node[i] < -1 || hint_node[i] >= N) return bad("hinted node out of range");
+  // runs of each candidate's own pods: consecutive pods of one spec and no hint (a hinted pod is a run of its own)
+  std::vector<int32_t> run_off, cand_run_off(n_cand + 1);
+  for (int c = 0; c < n_cand; ++c) {
+    cand_run_off[c] = (int32_t)run_off.size();
+    for (int k = cand_pod_off[c]; k < cand_pod_off[c + 1]; ++k) {
+      const int pod = cand_pods[k];
+      bool start = k == cand_pod_off[c];
+      if (!start) {
+        const int prev = cand_pods[k - 1];
+        start = e->h_pend_spec[pod] != e->h_pend_spec[prev] || (hint_node && (hint_node[pod] >= 0 || hint_node[prev] >= 0));
+      }
+      if (start) run_off.push_back(k);
+    }
+  }
+  const int runs = (int)run_off.size();
+  cand_run_off[n_cand] = runs;
+  run_off.push_back(n_pods);
+  // one blob, in 4-byte words; inputs first (one upload), then outputs and work arrays
+  auto words = [](size_t bytes) { return (bytes + 3) / 4; };
+  auto even = [](size_t w) { return (w + 1) & ~(size_t)1; };   // 8-byte alignment for the int64 / uint64 arrays
+  const int A1 = std::max(e->A, 1);
+  size_t off = 0;
+  const size_t o_st = off; off += cae::SIM_WORDS;
+  const size_t o_cand = off; off += n_cand;
+  const size_t o_poff = off; off += n_cand + 1;
+  const size_t o_pods = off; off += std::max(n_pods, 1);
+  const size_t o_run = off; off += runs + 1;
+  const size_t o_crun = off; off += n_cand + 1;
+  const size_t o_iota = off; off += P + 1;
+  const size_t o_hint = off; off += hint_node ? P : 0;
+  const size_t o_nodeok = off; off += node_ok ? words(N) : 0;
+  const size_t o_in_end = off;
+  const size_t o_res = off; off += n_cand;
+  const size_t o_toff = off; off += n_cand + 1;
+  const size_t o_tpod = off; off += std::max(trace_cap, 1);
+  const size_t o_tnode = off; off += std::max(trace_cap, 1);
+  const size_t o_out = off; off += 4;
+  const size_t o_pos = off; off += N;
+  const size_t o_at = off; off += N;
+  const size_t o_gone = off; off += n_cand;
+  const size_t o_mvt = off; off += N;
+  const size_t o_mvn = off; off += std::max(P, 1);
+  const size_t o_bksl = off; off += N;
+  const size_t o_zero = off;   // zeroed: seen, nok
+  const size_t o_seen = off; off += words(N);
+  const size_t o_nok = off; off += words(N);
+  const size_t o_ones = off;   // 0x01 bytes: present
+  const size_t o_pres = off; off += words(N);
+  const size_t o_mvh = off; off += N;   // 0xFF: -1
+  off = even(off);
+  const size_t o_bkp = off; off += (size_t)2 * N;
+  const size_t o_bkf = off; off += (size_t)2 * A1 * N;
+  if (off > e->fm_blob_words) {
+    if (e->d_fm_blob) cudaFree(e->d_fm_blob);
+    e->d_fm_blob = nullptr;
+    e->fm_blob_words = 0;
+    CAE_CUDA(cudaMalloc(&e->d_fm_blob, off * 4));
+    e->fm_blob_words = off;
+  }
+  std::vector<int32_t> hostblob(o_in_end, 0);
+  hostblob[o_st + cae::SIM_LI] = last_index_in;
+  std::copy(cand_node, cand_node + n_cand, hostblob.begin() + o_cand);
+  std::copy(cand_pod_off, cand_pod_off + n_cand + 1, hostblob.begin() + o_poff);
+  if (n_pods) std::copy(cand_pods, cand_pods + n_pods, hostblob.begin() + o_pods);
+  std::copy(run_off.begin(), run_off.end(), hostblob.begin() + o_run);
+  std::copy(cand_run_off.begin(), cand_run_off.end(), hostblob.begin() + o_crun);
+  for (int i = 0; i <= P; ++i) hostblob[o_iota + i] = i;
+  if (hint_node) std::copy(hint_node, hint_node + P, hostblob.begin() + o_hint);
+  if (node_ok && N) memcpy(hostblob.data() + o_nodeok, node_ok, N);
+  int32_t* blob = e->d_fm_blob;
+  CAE_CUDA(cudaMemcpyAsync(blob, hostblob.data(), o_in_end * 4, cudaMemcpyHostToDevice, e->stream));
+  CAE_CUDA(cudaMemsetAsync(blob + o_zero, 0, (o_ones - o_zero) * 4, e->stream));
+  CAE_CUDA(cudaMemsetAsync(blob + o_ones, 0x01, (o_mvh - o_ones) * 4, e->stream));
+  CAE_CUDA(cudaMemsetAsync(blob + o_mvh, 0xFF, (size_t)N * 4, e->stream));
+  CAE_CUDA(cudaMemsetAsync(blob + o_out, 0, 4 * 4, e->stream));
+  cae::SimLaunch s{};
+  s.n = n_cand; s.persist = persist ? 1 : 0; s.max_removable = max_removable; s.trace_cap = trace_cap;
+  s.cand = blob + o_cand; s.pod_off = blob + o_poff; s.pods = blob + o_pods; s.cand_run_off = blob + o_crun; s.iota = blob + o_iota;
+  s.result = blob + o_res; s.trace_off = blob + o_toff; s.trace_pod = blob + o_tpod; s.trace_node = blob + o_tnode; s.st = blob + o_st;
+  s.present = reinterpret_cast<uint8_t*>(blob + o_pres); s.nok = reinterpret_cast<uint8_t*>(blob + o_nok);
+  s.seen = reinterpret_cast<uint8_t*>(blob + o_seen);
+  s.pos = blob + o_pos; s.at = blob + o_at; s.gone = blob + o_gone;
+  s.mv_head = blob + o_mvh; s.mv_tail = blob + o_mvt; s.mv_next = blob + o_mvn; s.bk_slots = blob + o_bksl;
+  s.bk_free = reinterpret_cast<int64_t*>(blob + o_bkf); s.bk_ports = reinterpret_cast<unsigned long long*>(blob + o_bkp);
+  cae::FilterLaunch f{};
+  f.runs = runs; f.n_pods = trace_cap; f.last_index = last_index_in; f.break_on_failure = 1; f.nctrl = 0;
+  f.run_off = blob + o_run; f.pods = blob + o_pods;
+  f.hint = hint_node ? blob + o_hint : nullptr;
+  f.cls = nullptr; f.class_ctrl = blob + o_cand;   // no similarity classes: with breakOnFailure a mark never changes a result
+  f.node_ok = node_ok ? reinterpret_cast<const uint8_t*>(blob + o_nodeok) : nullptr;
+  f.assigned = nullptr; f.out = blob + o_out; f.ctrl_cnt = nullptr; f.class_mark = nullptr; f.ctrl_over = nullptr;
+  f.sim = &s;
+  cudaEventRecord(e->ev0, e->stream);
+  if (cae::launch_filter(e, f)) return -1;
+  cudaEventRecord(e->ev1, e->stream);
+  int32_t out[4] = {0, 0, 0, 0}, status = 0;
+  CAE_CUDA(cudaMemcpyAsync(result, blob + o_res, (size_t)n_cand * 4, cudaMemcpyDeviceToHost, e->stream));
+  CAE_CUDA(cudaMemcpyAsync(trace_off, blob + o_toff, (size_t)(n_cand + 1) * 4, cudaMemcpyDeviceToHost, e->stream));
+  CAE_CUDA(cudaMemcpyAsync(out, blob + o_out, sizeof(out), cudaMemcpyDeviceToHost, e->stream));
+  CAE_CUDA(cudaMemcpyAsync(&status, e->d_work_counter + 1, sizeof(int32_t), cudaMemcpyDeviceToHost, e->stream));
+  CAE_CUDA(cudaStreamSynchronize(e->stream));
+  float ms = 0;
+  cudaEventElapsedTime(&ms, e->ev0, e->ev1);
+  e->stats.estimate_ms = ms;
+  if (status == 2) { cae::set_error("cae_simulate_removals: the trace needs more than trace_cap entries"); return 1; }
+  if (status) { cae::set_error("placement log overflow in the filter pass"); return 1; }
+  const int tr_n = trace_off[n_cand];
+  if (tr_n > 0) {
+    CAE_CUDA(cudaMemcpyAsync(trace_pod, blob + o_tpod, (size_t)tr_n * 4, cudaMemcpyDeviceToHost, e->stream));
+    CAE_CUDA(cudaMemcpyAsync(trace_node, blob + o_tnode, (size_t)tr_n * 4, cudaMemcpyDeviceToHost, e->stream));
+    CAE_CUDA(cudaStreamSynchronize(e->stream));
+  }
+  *last_index_out = out[0];
+  return 0;
+}
+
 void* cae_stream(cae_engine* h) {
   Engine* e = reinterpret_cast<Engine*>(h);
   return e ? reinterpret_cast<void*>(e->stream) : nullptr;

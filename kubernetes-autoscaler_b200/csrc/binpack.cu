@@ -65,6 +65,19 @@ struct BpParams {
   int32_t *fm_assigned, *fm_out;          // [P] node or -1; {lastIndex, overflowing controllers, pods scheduled, moved}
   int32_t* fm_ctrl_cnt;                   // [controllers] classes stored per controller (zeroed)
   uint8_t *fm_class_mark, *fm_ctrl_over;  // [classes] known unschedulable, [controllers] overflowing (zeroed)
+  // batched scale-down (FM with sim_n > 0): RemovalSimulator.SimulateNodeRemoval for sim_n candidates in turn, see the kernel
+  int sim_n, sim_persist, sim_max_removable, sim_trace_cap;
+  const int32_t *sim_cand, *sim_pod_off, *sim_pods, *sim_run_off;   // [n] node, [n+1] own pods (CSR), [n+1] own runs in grec
+  const GroupRec* sim_rec_pod;            // [P] one-pod record of every pending pod (pods moved in by an earlier candidate)
+  int32_t *sim_result, *sim_trace_off, *sim_trace_pod, *sim_trace_node;
+  int32_t* sim_st;                             // [SIM_WORDS] state of the candidate loop (SIM_LI = lastIndex in, raw)
+  const uint8_t* sim_dest;                     // [N] destination map or NULL; fm_node_ok then points at sim_nok
+  uint8_t *sim_present, *sim_nok, *sim_seen;   // [N] node in the snapshot (init 1), present && destination, candidate seen
+  int32_t *sim_pos, *sim_at, *sim_gone;        // [N] list position of a present node, node at a position; [n] nodes taken out
+  int32_t *sim_mv_head, *sim_mv_tail, *sim_mv_next;   // pods placed on a node by persisted simulations, in placement order
+  int64_t* sim_bk_free;                        // [A1][N] node state before the running simulation (undo)
+  unsigned long long* sim_bk_ports;
+  int32_t* sim_bk_slots;
   unsigned char* scratch;
   size_t scratch_per_cta;
 };
@@ -213,6 +226,13 @@ __device__ __forceinline__ int bp_div_f(int64_t f, int64_t r, float rinv, int kb
 // pods arrive as runs of consecutive identical pods in the caller's order.  Plain runs are dealt in closed form (lap by lap,
 // because every pod's node is reported), hinted pods and pods under topology counters one by one, with the
 // SimilarPodsScheduling shortcut (similar_pods.go:59-104).
+// With p.sim_n > 0 the same block runs the planner's scale-down loop (RemovalSimulator.SimulateNodeRemoval per candidate,
+// simulator/cluster.go:126-217): candidates in order on one snapshot, each one's pods tried with breakOnFailure on the node
+// list WITHOUT the candidate.  The node list is the cluster order minus the nodes taken out (presence mask + block prefix:
+// scans and lastIndex use list positions); a taken-out node's residents and the pods logged on it stop counting and its
+// domains lose one eligible node (replayed into the copy-on-write counters like the placement log).  A successful
+// simulation with persist stays (its pods are appended to the pods-to-move of the nodes they landed on), any other one is
+// undone from a copy of the node state and by truncating the log.  lastIndex runs through the whole loop.
 template <int A, int TPB, bool WIN, bool FM>
 __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack_kernel(DevObjects o, DynTables d, BpParams p) {
   constexpr int NW = TPB / 32;
@@ -310,6 +330,12 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
       __syncthreads();
     };
     if (FM) ensure_cluster();
+    // batched scale-down: node list of the running simulation (identity for a single filter pass)
+    const bool batch = FM && p.sim_n > 0;
+    auto sv = [&](int i) -> int32_t& { return p.sim_st[i]; };   // state of the candidate loop (thread 0 writes, barriers publish)
+    auto Ncur = [&]() -> int { return batch ? sv(SIM_NCUR) : N; };   // length of the node list
+    auto pos_of = [&](int x) -> int { return batch ? p.sim_pos[x] : x; };
+    auto node_at = [&](int i) -> int { return batch ? p.sim_at[i] : i; };
     // Upper bounds of what ANY added node still has (free only shrinks, so a stale bound stays valid): a group whose
     // request exceeds them skips its pass over the open nodes; tightened whenever such a pass finds no room at all.
     int64_t maxfree[A1];
@@ -344,7 +370,10 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
       for (int a = 0; a < A; ++a) maxfree[a] = bp_wmax_ll(lane < NW ? S.rb[par][lane][a] : LLONG_MIN);
       par ^= 1;
     };
-    const int n_groups = FM ? p.fm_runs : p.order_n[t];
+    const int n_groups0 = FM ? p.fm_runs : p.order_n[t];
+    auto n_groups = [&]() -> int { return batch ? sv(SIM_RUNS_OWN) + sv(SIM_MOVED) : n_groups0; };
+    // pod k of the pass (batch: of the running simulation's list in the trace: its own pods, then the pods moved in)
+    auto run_pod = [&](int k) -> int { return batch ? p.sim_trace_pod[sv(SIM_SEG) + k] : p.fm_pods[k]; };
 
     auto log_append = [&](int x, int spec, int cnt) {  // any thread
       const int idx = atomicAdd(&S.log_n, 1);
@@ -499,20 +528,100 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
     const int32_t* order_row = FM ? nullptr : p.order + (size_t)t * p.E;   // FM: the runs in order
     auto fetch_rec = [&](int graw, int buf) {
       if (warp == 0) {
-        if (lane < 9) bp_cp_async16(reinterpret_cast<char*>(&S.rec[buf]) + lane * 16,
-                                    reinterpret_cast<const char*>(p.grec + (graw & ~ORDER_NOT_ON_FRESH)) + lane * 16);
+        const GroupRec* src = p.grec + (graw & ~ORDER_NOT_ON_FRESH);
+        if (batch) {   // the simulation's own runs, then one run per pod moved in
+          const int ro = sv(SIM_RUNS_OWN);
+          src = graw < ro ? p.grec + sv(SIM_RUN0) + graw : p.sim_rec_pod + run_pod(sv(SIM_OWN_N) + graw - ro);
+        }
+        if (lane < 9) bp_cp_async16(reinterpret_cast<char*>(&S.rec[buf]) + lane * 16, reinterpret_cast<const char*>(src) + lane * 16);
         bp_cp_async_commit();
       }
     };
-    int ord_cur = n_groups > 0 ? (FM ? 0 : order_row[0]) : 0, ord_next = n_groups > 1 ? (FM ? 1 : order_row[1]) : 0;
-    if (n_groups > 0) fetch_rec(ord_cur, 0);
+    // block-wide exclusive prefix of a per-node flag over x = 0..N-1 (ballots + one warp scan per TPB nodes); fn(x, rank)
+    // is called for every x < N with the flag set; returns the count
+    auto node_prefix = [&](auto flag, auto fn) -> int {
+      int basecnt = 0;
+      for (int base = 0; base < N; base += TPB) {
+        const int x = base + tid;
+        const bool ex = x < N && flag(x);
+        const unsigned mm = __ballot_sync(0xffffffffu, ex);
+        if (lane == 0) S.ri[par][warp][0] = __popc(mm);
+        __syncthreads();
+        const int v = lane < NW ? S.ri[par][lane][0] : 0;
+        int inc = v;
+#pragma unroll
+        for (int off = 1; off < 32; off <<= 1) {
+          const int u = __shfl_up_sync(0xffffffffu, inc, off);
+          if (lane >= off) inc += u;
+        }
+        const int wpre = __shfl_sync(0xffffffffu, inc - v, warp);
+        if (ex) fn(x, basecnt + wpre + __popc(mm & ((1u << lane) - 1)));
+        basecnt += __shfl_sync(0xffffffffu, inc, 31);
+        par ^= 1;
+      }
+      return basecnt;
+    };
+
+    for (;;) {   // candidates (a single filter pass runs once)
+    if (batch) {
+      // ---- next candidate: NoNodeInfo / not simulated / simulate (its pod list goes to the trace) ----
+      if (sv(SIM_CAND) >= p.sim_n) break;
+      __syncthreads();
+      if (tid == 0) {
+        const int cand = sv(SIM_CAND)++;
+        const int c = p.sim_cand[cand], own0 = p.sim_pod_off[cand], own_n = p.sim_pod_off[cand + 1] - own0, trn = sv(SIM_TRN);
+        int res = 3, moved = 0;   // 3 = simulate
+        if (sv(SIM_CUT)) res = -1;
+        else if (!p.sim_present[c] || p.sim_seen[c]) res = 2;   // removed by an earlier persisted simulation, or listed twice
+        else {
+          for (int q = p.sim_mv_head[c]; q >= 0; q = p.sim_mv_next[q]) ++moved;
+          if ((long long)trn + own_n + moved > p.sim_trace_cap) res = 4;   // trace capacity: nothing is guessed
+        }
+        p.sim_trace_off[cand] = trn;
+        if (res == 3) {
+          p.sim_seen[c] = 1;
+          p.sim_present[c] = 0;
+          p.sim_gone[sv(SIM_NREM)] = c;
+          int k = trn + own_n;   // pods placed on c by earlier persisted simulations follow its own pods, in placement order
+          for (int q = p.sim_mv_head[c]; q >= 0; q = p.sim_mv_next[q]) { p.sim_trace_pod[k] = q; p.sim_trace_node[k] = -1; ++k; }
+          sv(SIM_SEG) = trn; sv(SIM_TRN) = k;
+          sv(SIM_RUN0) = p.sim_run_off[cand]; sv(SIM_RUNS_OWN) = p.sim_run_off[cand + 1] - p.sim_run_off[cand];
+          sv(SIM_LOG0) = S.log_n;
+        } else if (res != 4) p.sim_result[cand] = res;
+        sv(SIM_RES) = res; sv(SIM_C) = c; sv(SIM_OWN0) = own0; sv(SIM_OWN_N) = own_n; sv(SIM_MOVED) = moved;
+      }
+      __syncthreads();
+      const int res = sv(SIM_RES);
+      if (res == 4) { if (tid == 0) atomicExch(p.status, 2); break; }
+      if (res != 3) continue;
+      {
+        const int seg = sv(SIM_SEG), own0 = sv(SIM_OWN0), own_n = sv(SIM_OWN_N);
+        for (int i = tid; i < own_n; i += TPB) { p.sim_trace_pod[seg + i] = p.sim_pods[own0 + i]; p.sim_trace_node[seg + i] = -1; }
+      }
+      // list positions of the nodes in the snapshot, and the node state to restore if the simulation does not stay
+      const int ncur = node_prefix([&](int x) { return p.sim_present[x] != 0; }, [&](int x, int r) { p.sim_pos[x] = r; p.sim_at[r] = x; });
+      for (int x = tid; x < N; x += TPB) {
+        p.sim_nok[x] = p.sim_present[x] && (!p.sim_dest || p.sim_dest[x]);   // read back through fm_node_ok
+#pragma unroll
+        for (int a = 0; a < A; ++a) p.sim_bk_free[(size_t)a * N + x] = g_free[(size_t)a * Xg + x];
+        p.sim_bk_slots[x] = g_slots[x];
+        p.sim_bk_ports[x] = g_ports[x];
+      }
+      const int li = sv(SIM_LI);   // raw: a scan starts at lastIndex % (current list length)
+      if (tid == 0) sv(SIM_NCUR) = ncur;
+      last_index = ncur > 0 ? (int)((((long long)li % ncur) + ncur) % ncur) : 0;
+      fm_moved = false; fm_stop = false; pods_total = 0;
+      __syncthreads();
+    }
+    int ord_cur = n_groups() > 0 ? (FM ? 0 : order_row[0]) : 0, ord_next = n_groups() > 1 ? (FM ? 1 : order_row[1]) : 0;
+    if (n_groups() > 0) fetch_rec(ord_cur, 0);
     if (warp == 0) bp_cp_async_wait();
     __syncthreads();
 
-    for (int gi = 0; gi < n_groups; ++gi) {
+    for (int gi = 0; gi < n_groups(); ++gi) {
       const GroupRec& rc = S.rec[gi & 1];
-      if (gi + 1 < n_groups) fetch_rec(ord_next, (gi + 1) & 1);
-      const int ord_next2 = gi + 2 < n_groups ? (FM ? gi + 2 : order_row[gi + 2]) : 0;
+      if (gi + 1 < n_groups()) fetch_rec(ord_next, (gi + 1) & 1);
+      const int ord_next2 = gi + 2 < n_groups() ? (FM ? gi + 2 : order_row[gi + 2]) : 0;
       const int g = ord_cur & ~ORDER_NOT_ON_FRESH;
       int n = rc.n;
       const int spec = rc.spec;
@@ -527,7 +636,8 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
       const unsigned long long pconf = rc.pconf;  // port sets this pod collides with
       const unsigned long long pbit = rc.pbit;
       const bool feeds = (rc.flags & GREC_FEEDS) != 0;
-      const int pb = rc.pad[0];   // FM: offset of the run in fm_pods
+      // FM: offset of the run in the pass's pod list (batch: own runs first, then the pods moved in, one run each)
+      const int pb = !batch ? rc.pad[0] : gi < sv(SIM_RUNS_OWN) ? rc.pad[0] - sv(SIM_OWN0) : sv(SIM_OWN_N) + gi - sv(SIM_RUNS_OWN);
       bool can_existing = n_new > 0 && static_new && maxslots >= 1;   // some added node may still take this pod
 #pragma unroll
       for (int a = 0; a < A; ++a) can_existing = can_existing && !(req[a] > 0 && req[a] > maxfree[a]);
@@ -634,7 +744,7 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
 
       // SimilarPodsScheduling (similar_pods.go:59-104): a pod that fitted nowhere marks its (controller, spec) class, at most
       // 10 classes per controller; later pods of a marked class are not tried
-      const int fm_cls = (FM && p.fm_class) ? p.fm_class[p.fm_pods[pb]] : -1;
+      const int fm_cls = (FM && p.fm_class) ? p.fm_class[run_pod(pb)] : -1;
       bool fm_blocked = FM && fm_cls >= 0 && p.fm_class_mark[fm_cls] != 0;
       auto fm_mark_failed = [&]() {
         if (fm_cls < 0) return;
@@ -648,11 +758,16 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
         if (cnt < 10) fm_blocked = true;
         __syncthreads();
       };
-      const int fm_hint = (FM && p.fm_hint) ? p.fm_hint[p.fm_pods[pb]] : -1;   // hinted pods are singleton runs
+      // hinted pods are singleton runs; a pod moved in was placed on the candidate itself, so its hint names a node out of the list
+      const int fm_hint = (FM && p.fm_hint && !(batch && gi >= sv(SIM_RUNS_OWN))) ? p.fm_hint[run_pod(pb)] : -1;
+      auto fm_set = [&](int k, int x) {   // node of pod k of the list (run_pod)
+        if (batch) p.sim_trace_node[sv(SIM_SEG) + k] = x;
+        else p.fm_assigned[p.fm_pods[k]] = x;
+      };
       // FM: deal m identical pods over the cluster nodes with capacities g_kc[x], lap by lap (lap l serves the nodes with
       // capacity >= l in cyclic order from lastIndex), reporting every pod's node; books the pods and moves lastIndex
       auto fm_deal = [&](int m) {
-        const int s = last_index < N ? last_index : 0;
+        const int s = node_at(last_index < Ncur() ? last_index : 0);
         for (int x = tid; x < N; x += TPB) g_aux[x] = 0;
         int done = 0, lap = 1;
         while (done < m) {
@@ -687,7 +802,7 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
             int rank = g_pre[x] - pre_s;
             if (x < s) rank += tot;
             if (rank < take) {
-              p.fm_assigned[p.fm_pods[pb + done + rank]] = x;
+              fm_set(pb + done + rank, x);
               g_aux[x] += 1;
               if (rank == take - 1) S.lastnode = x;
             }
@@ -698,7 +813,7 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
         }
         if (m > 0) {
           for (int x = tid; x < N; x += TPB) if (g_aux[x] > 0) book_c(x, g_aux[x]);
-          last_index = (S.lastnode + 1) % N;
+          last_index = (pos_of(S.lastnode) + 1) % Ncur();
           fm_moved = true;
           placed += m;
         }
@@ -706,7 +821,7 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
       };
       if (FM && dc == 0 && fm_hint < 0) {
         // ======================= plain run on the cluster nodes: dealt lap by lap ==================
-        if (fm_stop || fm_blocked || N == 0) {
+        if (fm_stop || fm_blocked || Ncur() == 0) {
           if (p.fm_break && n > 0) fm_stop = true;     // every pod of the run stays unschedulable (breakOnFailure, :71-73)
         } else {
           int total = 0, zero = 0, zero2 = 0;
@@ -737,19 +852,20 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
             where = h;
             placed += 1;
           }
-          if (where < 0 && !fm_blocked && N > 0) {   // SchedulePodOnAnyNodeMatching (:117): whole list, cyclic from lastIndex
+          if (where < 0 && !fm_blocked && Ncur() > 0) {   // SchedulePodOnAnyNodeMatching (:117): whole list, cyclic from lastIndex
             int best = INT_MAX, zero = 0;
             for (int x = tid; x < N; x += TPB) {
               if (o.node_unschedulable[x] || (p.fm_node_ok && !p.fm_node_ok[x]) || (p.pre_code[(size_t)sc * p.U + x] & 0x0F) != 0) continue;
-              if (res_cap_c(x, 1) > 0) { int dd = x - last_index; if (dd < 0) dd += N; best = min(best, dd); }
+              if (res_cap_c(x, 1) > 0) { int dd = pos_of(x) - last_index; if (dd < 0) dd += Ncur(); best = min(best, dd); }
             }
             blk_min_sum<NW>(S, par, best, zero);
             if (best != INT_MAX) {
-              int hit = last_index + best;
-              if (hit >= N) hit -= N;
+              int hpos = last_index + best;
+              if (hpos >= Ncur()) hpos -= Ncur();
+              const int hit = node_at(hpos);
               if (tid == 0) book_c(hit, 1);
               __syncthreads();
-              last_index = (hit + 1) % N;
+              last_index = (hpos + 1) % Ncur();
               fm_moved = true;
               where = hit;
               placed += 1;
@@ -757,7 +873,7 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
           }
           if (where < 0 && p.fm_break) fm_stop = true;
         }
-        if (tid == 0) p.fm_assigned[p.fm_pods[pb]] = where;
+        if (tid == 0) fm_set(pb, where);
       } else if (dc == 0) {
         // ======================= plain group: closed form =======================================
         BP_PROF_COUNT(8, 1);
@@ -923,19 +1039,26 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
         __syncthreads();
         run_flagged();
         const bool need_log = S.need_log != 0;
-        // ---- then the run's placement log if other groups feed us ----
-        if (need_log && S.log_n > 0) {
+        // ---- then the run's placement log if other groups feed us, and (batch) the nodes out of the list ----
+        if ((need_log && S.log_n > 0) || batch) {
           const int nlog = min(S.log_n, p.log_cap);
           for (int q = 0; q < nq; ++q) {
             const int qid = wd.qid[q];
             // Pass 1 materialises the touched copy-on-write slots with their defaults (identical values from
-            // every thread), pass 2 stamps the version and adds the weights atomically.
+            // every thread), pass 2 stamps the version and adds the weights atomically.  Batch: a placement logged on a
+            // node out of the list no longer counts; a node out of the list takes its residents' weights and one eligible
+            // node from its domain.
             int touched = 0;
             long long dt = 0;
+            auto gone_w = [&](int x) -> int {
+              int w = 0;
+              for (int r = o.node_pod_off[x]; r < o.node_pod_off[x + 1]; ++r) w += d.wmat[(size_t)qid * d.S + o.node_pod_spec[r]];
+              return w;
+            };
             for (int i = tid; i < nlog; i += TPB) {
               const int x = logbuf[i * 3];
               const int w = d.wmat[(size_t)qid * d.S + logbuf[i * 3 + 1]];
-              if (w == 0 || !elig_of(q, x)) continue;
+              if (w == 0 || !elig_of(q, x) || (batch && !p.sim_present[x])) continue;
               const int sl = slot_of(q, x);
               if (sl < 0) continue;
               const size_t o2 = (size_t)q * p.dstride + sl;
@@ -943,21 +1066,44 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
               touched = 1;
               dt += w * logbuf[i * 3 + 2];
             }
+            if (batch) {
+              for (int i = tid; i <= sv(SIM_NREM); i += TPB) {   // the removed nodes, then the candidate
+                const int x = p.sim_gone[i];
+                if (!elig_of(q, x)) continue;
+                const int sl = slot_of(q, x);
+                if (sl < 0) continue;
+                const size_t o2 = (size_t)q * p.dstride + sl;
+                if (wver[o2] != gver) { wcnt[o2] = def_cnt(q, sl); wpres[o2] = def_pres(q, sl); }
+                dt -= gone_w(x);
+              }
+            }
             __syncthreads();
             for (int i = tid; i < nlog; i += TPB) {
               const int x = logbuf[i * 3];
               const int w = d.wmat[(size_t)qid * d.S + logbuf[i * 3 + 1]];
-              if (w == 0 || !elig_of(q, x)) continue;
+              if (w == 0 || !elig_of(q, x) || (batch && !p.sim_present[x])) continue;
               const int sl = slot_of(q, x);
               if (sl < 0) continue;
               const size_t o2 = (size_t)q * p.dstride + sl;
               wver[o2] = gver;
               atomicAdd(&wcnt[o2], w * logbuf[i * 3 + 2]);
             }
+            if (batch) {
+              for (int i = tid; i <= sv(SIM_NREM); i += TPB) {   // the removed nodes, then the candidate
+                const int x = p.sim_gone[i];
+                if (!elig_of(q, x)) continue;
+                const int sl = slot_of(q, x);
+                if (sl < 0) continue;
+                const size_t o2 = (size_t)q * p.dstride + sl;
+                wver[o2] = gver;
+                atomicAdd(&wcnt[o2], -gone_w(x));
+                atomicAdd(&wpres[o2], -1);
+              }
+            }
             blk_sum_ll_max<NW>(S, par, dt, touched);
             if (tid == 0) wd.tot[q] += (int)dt;
             __syncthreads();
-            if (touched > 0 && wd.kind[q] == Q_PTS) recompute(q);
+            if ((touched > 0 || batch) && wd.kind[q] == Q_PTS) recompute(q);
           }
         }
 
@@ -1069,7 +1215,7 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
               h_caps(x, cp, ci);
               const int k_other = min(rc, ci);
               g_kc[x] = min(k_other, cp);
-              if (k_other == 0 && hp >= 0) {
+              if (k_other == 0 && hp >= 0 && !(batch && !p.sim_present[x])) {
                 const int sl = slot_of(hp, x);
                 if (sl >= 0 && elig_of(hp, x) && rd_cnt(hp, sl) == 0 && rd_pres(hp, sl) == 1) blocked = 1;
               }
@@ -1080,11 +1226,11 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
             BP_PROF_COUNT(14, 1);
             return blocked > 0;
           };
-          if (ok && hp >= 0 && !(wd.wown[hp] == 0 || wd.nmin[hp] > n)) ok = N > 0 ? cluster_caps() : false;   // is the minimum pinned?
+          if (ok && hp >= 0 && !(wd.wown[hp] == 0 || wd.nmin[hp] > n)) ok = Ncur() > 0 ? cluster_caps() : false;   // is the minimum pinned?
           if (FM && ok) {
             // hostname counters only: per-node capacities over the cluster nodes, dealt like a plain run
             fast = true;
-            if (fm_stop || fm_blocked || N == 0) {
+            if (fm_stop || fm_blocked || Ncur() == 0) {
               if (p.fm_break && n > 0) fm_stop = true;
             } else {
               if (!caps_done) cluster_caps();
@@ -1321,24 +1467,24 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
           const int run_n = n;
           bool run_failed = false;  // a pod of this run fitted nowhere: the identical pods behind it see the same state
           for (int i = 0; i < run_n; ++i) {
-            const int pod = p.fm_pods[pb + i];
             int where = -1;
             if (!fm_stop) {
-              const int h = p.fm_hint ? p.fm_hint[pod] : -1;   // tryScheduleUsingHints (:80-106); lastIndex untouched
+              const int h = fm_hint;   // tryScheduleUsingHints (:80-106); lastIndex untouched.  Only singleton runs carry a hint
               if (h >= 0 && h < N && (!p.fm_node_ok || p.fm_node_ok[h]) && eval(h) == CAE_R_OK) { place(h); where = h; }
-              if (where < 0 && !fm_blocked && !run_failed && N > 0) {
+              if (where < 0 && !fm_blocked && !run_failed && Ncur() > 0) {
                 // SchedulePodOnAnyNodeMatching (:117): whole list, cyclic from lastIndex
                 int best = INT_MAX, zero = 0;
                 for (int x = tid; x < N; x += TPB) {
                   if (o.node_unschedulable[x] || (p.fm_node_ok && !p.fm_node_ok[x])) continue;
-                  if (eval(x) == CAE_R_OK) { int dd = x - last_index; if (dd < 0) dd += N; best = min(best, dd); }
+                  if (eval(x) == CAE_R_OK) { int dd = pos_of(x) - last_index; if (dd < 0) dd += Ncur(); best = min(best, dd); }
                 }
                 blk_min_sum<NW>(S, par, best, zero);
                 if (best != INT_MAX) {
-                  int hit = last_index + best;
-                  if (hit >= N) hit -= N;
+                  int hpos = last_index + best;
+                  if (hpos >= Ncur()) hpos -= Ncur();
+                  const int hit = node_at(hpos);
                   place(hit);
-                  last_index = (hit + 1) % N;
+                  last_index = (hpos + 1) % Ncur();
                   fm_moved = true;
                   where = hit;
                 } else {
@@ -1348,7 +1494,7 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
               }
               if (where < 0 && p.fm_break) fm_stop = true;   // breakOnFailure (:71-73)
             }
-            if (tid == 0) p.fm_assigned[pod] = where;
+            if (tid == 0) fm_set(pb + i, where);
           }
         } else {
         // ---- tryToScheduleOnExistingNodes: per pod, first passing added node in cyclic order ----
@@ -1418,13 +1564,49 @@ __global__ void __launch_bounds__(TPB, FM ? 1 : BP_MIN_CTAS * 256 / TPB) binpack
       __syncthreads();
       ord_cur = ord_next;
       ord_next = ord_next2;
+      if (batch && fm_stop) break;         // breakOnFailure: the pods behind stay unplaced (-1 in the trace)
     }
+    if (batch) {
+      // ---- end of the candidate: removable iff every pod was placed; keep it (persist) or undo it ----
+      const bool removable = pods_total == sv(SIM_OWN_N) + sv(SIM_MOVED);
+      if (removable && p.sim_persist) {
+        if (tid == 0) {   // the pods now live where they were placed: append them there, in placement order
+          p.sim_mv_head[sv(SIM_C)] = -1;
+          for (int k = sv(SIM_SEG); k < sv(SIM_TRN); ++k) {
+            const int q = p.sim_trace_pod[k], x = p.sim_trace_node[k];
+            p.sim_mv_next[q] = -1;
+            if (p.sim_mv_head[x] < 0) p.sim_mv_head[x] = q;
+            else p.sim_mv_next[p.sim_mv_tail[x]] = q;
+            p.sim_mv_tail[x] = q;
+          }
+          sv(SIM_NREM) += 1;
+        }
+      } else {
+        for (int x = tid; x < N; x += TPB) {
+#pragma unroll
+          for (int a = 0; a < A; ++a) g_free[(size_t)a * Xg + x] = p.sim_bk_free[(size_t)a * N + x];
+          g_slots[x] = p.sim_bk_slots[x];
+          g_ports[x] = p.sim_bk_ports[x];
+        }
+        if (tid == 0) { S.log_n = sv(SIM_LOG0); p.sim_present[sv(SIM_C)] = 1; }
+      }
+      if (tid == 0) {
+        if (fm_moved) sv(SIM_LI) = last_index;   // the runner's lastIndex survives the revert
+        p.sim_result[sv(SIM_CAND) - 1] = removable ? 0 : 1;
+        if (removable && ++sv(SIM_NREMOVABLE) == p.sim_max_removable) sv(SIM_CUT) = 1;   // unneededNodesLimit
+      }
+      __syncthreads();
+    }
+    if (!batch) break;
+    }  // candidates
     if (p.prof && tid == 0) atomicAdd((unsigned long long*)&p.prof[7], (unsigned long long)(clock64() - prof_tmpl0));
     if constexpr (FM) {
       int over = 0, zero = 0;
       for (int c = tid; c < p.fm_nctrl; c += TPB) over += p.fm_ctrl_over[c] != 0;
       blk_sum_max<NW>(S, par, over, zero);
+      if (batch && tid == 0 && !p.status[0]) p.sim_trace_off[p.sim_n] = sv(SIM_TRN);
       if (tid == 0) {
+        if (batch) { last_index = sv(SIM_LI); fm_moved = true; }
         p.fm_out[0] = last_index; p.fm_out[1] = over; p.fm_out[2] = pods_total; p.fm_out[3] = fm_moved ? 1 : 0;
         if (S.overflow && p.status) atomicExch(p.status, 1);
       }
@@ -1636,11 +1818,13 @@ int launch_filter(Engine* e, const FilterLaunch& f) {
   int dmax = 1;
   for (int k = 0; k < e->dyn.K; ++k) dmax = std::max(dmax, e->dyn.Dc[k] + 2);
   p.dstride = p.has_dyn ? dmax : 1;
-  p.log_cap = p.has_dyn ? f.n_pods + 1024 : 1;   // one entry per placement at most
+  // one entry per placement at most (batch: per placement of the kept simulations and the running one, <= the trace)
+  p.log_cap = p.has_dyn ? f.n_pods + 1024 : 1;
   size_t per_cta = 16 + Xg * ((size_t)A1 * 8 + 8 + 4 + 4 + 4 + 4) + (size_t)3 * DYN_MAX_Q * p.dstride * 4 + (size_t)p.log_cap * 12 + Xg;
   per_cta = (per_cta + 255) & ~(size_t)255;
   p.scratch_per_cta = per_cta;
-  const size_t rec_bytes = ((size_t)std::max(f.runs, 1) * sizeof(GroupRec) + 255) & ~(size_t)255;
+  const int n_rec = f.runs + (f.sim ? e->P : 0);   // batch: + one record per pending pod
+  const size_t rec_bytes = ((size_t)std::max(n_rec, 1) * sizeof(GroupRec) + 255) & ~(size_t)255;
   const size_t need = per_cta + rec_bytes;
   const size_t sig = per_cta * 1000003u + Xg * 10007u + (size_t)p.dstride * 101u + (size_t)p.log_cap * 7u + (size_t)A1 + 0x7000000000ull;
   if (need > e->fm_scratch_bytes) {
@@ -1659,10 +1843,30 @@ int launch_filter(Engine* e, const FilterLaunch& f) {
   GroupRec* d_rec = reinterpret_cast<GroupRec*>(p.scratch + per_cta);
   p.grec = d_rec;
   CAE_CUDA(cudaMemsetAsync(e->d_work_counter, 0, sizeof(int32_t) * 2, e->stream));
-  run_rec_kernel<<<(f.runs + 127) / 128, 128, 0, e->stream>>>(e->dobj, e->dyn, f.runs, f.run_off, f.pods, e->A, e->d_act_dim, p.has_dyn,
-                                                             e->d_spec_sc, e->d_spec_dc, e->d_pc_of, e->d_port_conf, d_rec);
+  if (f.runs > 0) {
+    run_rec_kernel<<<(f.runs + 127) / 128, 128, 0, e->stream>>>(e->dobj, e->dyn, f.runs, f.run_off, f.pods, e->A, e->d_act_dim, p.has_dyn,
+                                                               e->d_spec_sc, e->d_spec_dc, e->d_pc_of, e->d_port_conf, d_rec);
+    e->stats.kernel_launches++;
+  }
+  if (const SimLaunch* s = f.sim) {
+    if (e->P > 0) {
+      run_rec_kernel<<<(e->P + 127) / 128, 128, 0, e->stream>>>(e->dobj, e->dyn, e->P, s->iota, s->iota, e->A, e->d_act_dim, p.has_dyn,
+                                                                e->d_spec_sc, e->d_spec_dc, e->d_pc_of, e->d_port_conf, d_rec + f.runs);
+      e->stats.kernel_launches++;
+    }
+    p.sim_n = s->n; p.sim_persist = s->persist; p.sim_max_removable = s->max_removable; p.sim_trace_cap = s->trace_cap;
+    p.sim_cand = s->cand; p.sim_pod_off = s->pod_off; p.sim_pods = s->pods; p.sim_run_off = s->cand_run_off;
+    p.sim_rec_pod = d_rec + f.runs;
+    p.sim_result = s->result; p.sim_trace_off = s->trace_off; p.sim_trace_pod = s->trace_pod; p.sim_trace_node = s->trace_node;
+    p.sim_st = s->st; p.sim_present = s->present; p.sim_nok = s->nok; p.sim_seen = s->seen;
+    p.sim_dest = f.node_ok;
+    p.fm_node_ok = s->nok;
+    p.sim_pos = s->pos; p.sim_at = s->at; p.sim_gone = s->gone;
+    p.sim_mv_head = s->mv_head; p.sim_mv_tail = s->mv_tail; p.sim_mv_next = s->mv_next;
+    p.sim_bk_free = s->bk_free; p.sim_bk_ports = s->bk_ports; p.sim_bk_slots = s->bk_slots;
+  }
   { int unused = 0; if (launch_binpack_any(e, 1, 0, p, &unused, false, true)) return -1; }
-  e->stats.kernel_launches += 2;
+  e->stats.kernel_launches++;
   CAE_KERNEL_OK();
   return 0;
 }

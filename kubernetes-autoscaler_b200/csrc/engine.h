@@ -193,12 +193,28 @@ int launch_group_feasibility(Engine* e);
 int launch_order(Engine* e);
 int launch_group_records(Engine* e);     // GroupRec[E] (after the class / counter tables of a load)
 int launch_binpack(Engine* e);   // K3: block-per-template estimator (binpack.cu)
+// cae_simulate_removals: the candidate loop of the filter pass (device pointers into the call's blob, see BpParams).
+// Words of SimLaunch::st: the running candidate and what the candidate loop carries (kept in global memory: the filter
+// instantiation of the kernel is at its register budget).  The caller zeroes them and sets SIM_LI to the raw lastIndex.
+enum { SIM_RES, SIM_C, SIM_OWN0, SIM_OWN_N, SIM_MOVED, SIM_SEG, SIM_RUN0, SIM_RUNS_OWN, SIM_LOG0, SIM_NREM, SIM_TRN, SIM_LI,
+       SIM_NREMOVABLE, SIM_CUT, SIM_NCUR, SIM_CAND, SIM_WORDS };
+struct SimLaunch {
+  int n, persist, max_removable, trace_cap;
+  const int32_t *cand, *pod_off, *pods, *cand_run_off;
+  const int32_t* iota;   // [P + 1] 0, 1, ..., P: run offsets and pods of the one-pod records
+  int32_t *result, *trace_off, *trace_pod, *trace_node, *st;
+  uint8_t *present, *nok, *seen;
+  int32_t *pos, *at, *gone, *mv_head, *mv_tail, *mv_next, *bk_slots;
+  int64_t* bk_free;
+  unsigned long long* bk_ports;
+};
 struct FilterLaunch {
   int runs, n_pods, last_index, break_on_failure, nctrl;
   const int32_t *run_off, *pods, *hint, *cls, *class_ctrl;
   const uint8_t* node_ok;
   int32_t *assigned, *out, *ctrl_cnt;
   uint8_t *class_mark, *ctrl_over;
+  const SimLaunch* sim;   // NULL = one pass (cae_filter_schedulable)
 };
 int launch_filter(Engine* e, const FilterLaunch& f);
 int launch_price(Engine* e, const cae_price_inputs& in_dev, const int32_t* d_node_count, const int32_t* d_sched, const int32_t* d_order,

@@ -267,6 +267,38 @@ class Engine:
                                                     vp(assigned), vp(li), vp(ov)))
         return assigned[:enc.P], int(li[0]), int(ov[0])
 
+    def simulate_removals(self, cand_node: Sequence[int], cand_pod_off: Sequence[int], cand_pods: Sequence[int], hint_node=None,
+                          node_ok=None, persist: bool = True, max_removable: int = 0, last_index: int = 0,
+                          trace_cap: Optional[int] = None):
+        """RemovalSimulator.SimulateNodeRemoval for every candidate in turn on the snapshot of the last load
+        (cae_simulate_removals).  Returns (result[n_cand], trace_off[n_cand+1], trace_pod, trace_node, lastIndex afterwards).
+        The trace buffers start at `trace_cap` entries (default: twice the pods listed) and grow once, to the size no trace
+        can exceed, when the engine answers that they are too small."""
+        P = self.enc.P
+        cn = np.ascontiguousarray(cand_node, np.int32)
+        off = np.ascontiguousarray(cand_pod_off, np.int32)
+        pods = np.ascontiguousarray(cand_pods, np.int32)
+        hn = None if hint_node is None else np.ascontiguousarray(hint_node, np.int32)
+        ok = None if node_ok is None else np.ascontiguousarray(node_ok, np.uint8)
+        n = len(cn)
+        cap = 2 * len(pods) + 64 if trace_cap is None else int(trace_cap)
+        result = np.zeros(max(n, 1), np.int32)
+        toff = np.zeros(n + 1, np.int32)
+        li = np.zeros(1, np.int32)
+        vp = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+        for attempt in range(2):
+            tpod, tnode = np.zeros(max(cap, 1), np.int32), np.zeros(max(cap, 1), np.int32)
+            rc = self.lib.cae_simulate_removals(self.h, n, vp(cn), vp(off), vp(pods), vp(hn), vp(ok), int(bool(persist)),
+                                                int(max_removable), int(last_index), vp(result), cap, vp(toff), vp(tpod), vp(tnode),
+                                                vp(li))
+            if rc == 1 and attempt == 0 and b"trace" in (self.lib.cae_last_error() or b""):
+                cap = max(2 * cap, n * P)   # every simulated list holds distinct pending pods
+                continue
+            self._check(rc)
+            break
+        k = int(toff[n])
+        return result[:n], toff, tpod[:k], tnode[:k], int(li[0])
+
     # ---- fused histogram exchange over peer memory (multi-GPU dense pass) -------------------------
     def peer_handle(self) -> bytes:
         buf = C.create_string_buffer(capi.CONST["CAE_PEER_HANDLE_BYTES"])

@@ -6,8 +6,9 @@ self-cleaning accumulators, last-block election, shared-memory state and block-w
     compute-sanitizer --tool racecheck python scripts/sanitize.py
 
 Dense pass (K1, both variants), Estimate() of every template (K0 + K3: plain closed form, capacity form with the cluster
-fallback, per-pod loop), expander scores, the filter-out-schedulable pass — on miniatures of C2, C3 and C4 — each checked
-against the CPU oracle so that a "clean" run also means "correct results under the tool"."""
+fallback, per-pod loop), expander scores, the filter-out-schedulable pass — on miniatures of C2, C3 and C4 — and the batched
+scale-down loop (cae_simulate_removals), each checked against the CPU oracle so that a "clean" run also means "correct results
+under the tool"."""
 import os
 import sys
 
@@ -43,8 +44,21 @@ def main():
             ref = pyoracle.filter_schedulable(enc, order_p)
             assert np.array_equal(got[0], ref[0]) and got[1:] == ref[1:]
         print("config", cfg, "ok: nodes", int(nc.sum()), "pods", int(pc.sum()), flush=True)
+    removal_batch(eng)
     eng.close()
     print("sanitize workload ok")
+
+
+def removal_batch(eng):
+    """The batched scale-down loop (cae_simulate_removals: candidate loop, undo, persisted removals, pods moved again) on a
+    small cluster with topology spread and anti-affinity, checked against the sequential SimulateNodeRemoval loop."""
+    import copy
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
+    from test_removal_batch import _rand_scenario, check_batch
+    for seed in range(6):
+        cluster, cands, dest, persist, max_removable, hints, li = _rand_scenario(90_000 + seed)
+        check_batch(eng, copy.deepcopy(cluster), cands, dest, persist, max_removable, hints, li)
+    print("removal batch ok", flush=True)
 
 
 if __name__ == "__main__":
